@@ -14,7 +14,10 @@ The backbone / heads between those ops are cuDNN / cuBLAS work outside the scope
 step is captured in CUDA graphs; before timing, its outputs are checked once against the oracle.  The inference hot path
 of configs[1] (last round's headline) is kept as `extra.inference_hot_path`.  Prints ONE JSON line (DESIGN.md section 5).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the last timed step returned (rank 0) as DIR/<name>.npy, so that two builds can be compared
+output for output on the same seeded inputs (see dump_step_outputs).
 """
 import argparse
 import json
@@ -347,6 +350,46 @@ def validate_step(runner, d_host, d_dev, outs):
     return rep
 
 
+DUMP_SAMPLE = 1 << 17  # elements stored of a larger output
+
+
+def dump_step_outputs(outs, out_dir):
+    """Write the outputs of one TrainRunner.step as out_dir/<name>.npy: floating-point outputs in float32, kept indices and
+    counts in float64 (exact).  An output of more than DUMP_SAMPLE elements is stored as the 1-D sample of DUMP_SAMPLE
+    elements at fixed positions of its flattened (logical, row-major) order: torch.randperm with seed 0, sorted.  The
+    positions depend only on the output's size, so every build stores the same elements.  Returns the bytes written."""
+    import numpy as np
+
+    arrays = {}
+    for i, (keep, num) in enumerate(outs["keep"]):
+        arrays["rpn_nms_keep_img%d" % i] = keep[: int(num.item())]
+        arrays["rpn_nms_num_kept_img%d" % i] = num
+    arrays["box_pool_fwd"], arrays["mask_pool_fwd"] = outs["box"], outs["mask"]
+    for l, g in enumerate(outs["gfeat"]):
+        arrays["feature_grad_p%d" % (l + 2)] = g
+    k = 0
+    for c, _, _, layers in DCONV_STAGES:
+        for li in range(layers):
+            y, (gx, goff, _, gw, _) = outs["dc"][k]
+            for name, t in (("out", y), ("grad_x", gx), ("grad_offset", goff), ("grad_weight", gw)):
+                arrays["dconv_c%d_layer%d_%s" % (c, li, name)] = t
+            k += 1
+    os.makedirs(out_dir, exist_ok=True)
+    total, positions = 0, {}
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > DUMP_SAMPLE:
+            if t.numel() not in positions:
+                perm = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))
+                positions[t.numel()] = perm[:DUMP_SAMPLE].sort().values.to(t.device)
+            t = t.reshape(-1)[positions[t.numel()]]
+        a = t.cpu().numpy().astype(np.float32 if t.is_floating_point() else np.float64)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+        total += a.nbytes
+    assert total <= 64 << 20, total
+    return total
+
+
 # ----------------------------------------------------------------------------------------- inference hot path (extra)
 class InferenceRunner:
     def __init__(self, device):
@@ -543,7 +586,11 @@ def main():
     ap.add_argument("--steps", type=int, default=40)
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step (rank 0, impl ours) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -620,6 +667,9 @@ def main():
     barrier()
     sampler.active = False
     elapsed_ms = t_start.elapsed_time(t_end)
+    if args.dump_outputs and rank == 0:
+        # the last timed replay was graphs[(steps - 1) % NBUF]; its outputs live in that graph's static buffers
+        dump_step_outputs(graph_outs[(args.steps - 1) % NBUF], args.dump_outputs)
     del graphs, graph_outs
 
     # ---------------- per-stage device time: each stage captured alone in its own graphs, rotating inputs

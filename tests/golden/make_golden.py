@@ -1,16 +1,18 @@
 """Generate the committed golden fixtures (tests/golden/*.npz) from the REAL reference.
 
-Run in the authoring container only (needs /root/reference and torchvision):
-    python tests/golden/make_golden.py
+Needs a detectron2 source checkout (DETECTRON2_REFERENCE) and torchvision:
+    DETECTRON2_REFERENCE=<detectron2 checkout> python tests/golden/make_golden.py [fixture ...]
+With fixture names (e.g. `compiled_reference`), only those fixtures are rewritten.
 
 Sources of truth used (never our own code):
   * torchvision CPU ops  -- the reference's backend for roi_align / nms / deform_conv2d
     (detectron2/layers/roi_align.py:3,58; nms.py:5-22; deform_conv.py:9,55)
   * oracle/_ref/d2_ref_cpu.so -- the reference CPU csrc compiled in place (oracle/build.py):
     torch.ops.detectron2.{roi_align_rotated_forward,roi_align_rotated_backward,box_iou_rotated,nms_rotated}
-  * /root/reference/detectron2/layers/mask_ops.py loaded as a stand-alone module
+  * detectron2/layers/mask_ops.py of the checkout loaded as a stand-alone module
     (paste_masks_in_image, pure torch)
-Inputs are seeded; both inputs and outputs are stored so the GPU box needs nothing but the .npz.
+  * detectron2/layers/deform_conv.py of the checkout: the calls its autograd Functions make into `detectron2._C`
+Inputs are seeded; both inputs and outputs are stored so the tests need nothing but the .npz.
 """
 import importlib.util
 import os
@@ -23,6 +25,7 @@ from torchvision.ops import boxes as tv_boxes
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
+REF = os.environ["DETECTRON2_REFERENCE"]
 sys.path.insert(0, ROOT)
 from oracle import oracle as orc  # noqa: E402  (only for load_reference())
 
@@ -189,7 +192,7 @@ def gen_deform_conv():
 
 
 def gen_paste_masks():
-    spec = importlib.util.spec_from_file_location("ref_mask_ops", "/root/reference/detectron2/layers/mask_ops.py")
+    spec = importlib.util.spec_from_file_location("ref_mask_ops", REF + "/detectron2/layers/mask_ops.py")
     mo = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(mo)
     g = torch.Generator().manual_seed(42)
@@ -216,7 +219,7 @@ def _import_reference_proposal_utils():
         sys.modules[name] = m
         return m
 
-    sys.path.insert(0, "/root/reference")
+    sys.path.insert(0, REF)
     fv = stub("fvcore", __version__="0.1.5")
     fv.__path__ = []
     nn_ = stub("fvcore.nn")
@@ -227,7 +230,7 @@ def _import_reference_proposal_utils():
     pc.__path__ = []
     stub("pycocotools.mask")
     spec = importlib.util.spec_from_file_location(
-        "ref_proposal_utils", "/root/reference/detectron2/modeling/proposal_generator/proposal_utils.py")
+        "ref_proposal_utils", REF + "/detectron2/modeling/proposal_generator/proposal_utils.py")
     m = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(m)
     return m
@@ -284,7 +287,7 @@ def _import_reference_fast_rcnn():
     mm = stub("detectron2.modeling")
     mm.__path__ = []
     stub("detectron2.modeling.box_regression", Box2BoxTransform=object, _dense_box_regression_loss=None)
-    spec = importlib.util.spec_from_file_location("ref_fast_rcnn", "/root/reference/detectron2/modeling/roi_heads/fast_rcnn.py")
+    spec = importlib.util.spec_from_file_location("ref_fast_rcnn", REF + "/detectron2/modeling/roi_heads/fast_rcnn.py")
     m = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(m)
     return m
@@ -329,7 +332,7 @@ def _import_reference_dense_detector():
     mm = sys.modules["detectron2.modeling"]
     mm.Backbone = object
     spec = importlib.util.spec_from_file_location("detectron2.modeling.box_regression",
-                                                  "/root/reference/detectron2/modeling/box_regression.py")
+                                                  REF + "/detectron2/modeling/box_regression.py")
     br = importlib.util.module_from_spec(spec)
     sys.modules["detectron2.modeling.box_regression"] = br
     spec.loader.exec_module(br)
@@ -337,7 +340,7 @@ def _import_reference_dense_detector():
     ma.__path__ = []
     stub("detectron2.modeling.postprocessing", detector_postprocess=None)
     spec = importlib.util.spec_from_file_location("detectron2.modeling.meta_arch.dense_detector",
-                                                  "/root/reference/detectron2/modeling/meta_arch/dense_detector.py")
+                                                  REF + "/detectron2/modeling/meta_arch/dense_detector.py")
     dd = importlib.util.module_from_spec(spec)
     sys.modules["detectron2.modeling.meta_arch.dense_detector"] = dd
     spec.loader.exec_module(dd)
@@ -348,7 +351,7 @@ def gen_retinanet_inference():
     """RetinaNet.forward_inference (meta_arch/retinanet.py:256-308) on the real DenseDetector decode methods."""
     import types
 
-    dd, br = _import_reference_dense_detector()  # also puts /root/reference on sys.path
+    dd, br = _import_reference_dense_detector()  # also puts the reference checkout on sys.path
     from detectron2.layers import batched_nms
     from detectron2.structures import Boxes
 
@@ -391,7 +394,7 @@ def gen_postprocessing():
     _import_reference_fast_rcnn()  # stubs + sys.path
     from detectron2.structures import BitMasks, Boxes, Instances
 
-    spec = importlib.util.spec_from_file_location("ref_postprocessing", "/root/reference/detectron2/modeling/postprocessing.py")
+    spec = importlib.util.spec_from_file_location("ref_postprocessing", REF + "/detectron2/modeling/postprocessing.py")
     pp = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(pp)
     g = torch.Generator().manual_seed(808)
@@ -425,15 +428,153 @@ def gen_postprocessing():
     save("postprocessing", **out)
 
 
+def gen_compiled_reference():
+    """box_iou_rotated / nms_rotated and roi_align_rotated forward + backward of the compiled reference csrc, at the inputs of
+    the cross-checks in tests/test_oracle_pins.py (test_live_vs_compiled_reference, test_sweep_roi_align_rotated_*)."""
+    g = torch.Generator().manual_seed(11)
+    n = 150
+    b = torch.stack([torch.rand(n, generator=g) * 80, torch.rand(n, generator=g) * 80, 1 + torch.rand(n, generator=g) * 40,
+                     1 + torch.rand(n, generator=g) * 40, (torch.rand(n, generator=g) - 0.5) * 400], 1)
+    out = {"b": b, "ious": D2.box_iou_rotated(b, b.flip(0))}
+    out["s"] = s = torch.rand(n, generator=g)
+    out["thr"] = thrs = np.asarray([0.2, 0.5])
+    for i, thr in enumerate(thrs):
+        out[f"keep{i}"] = D2.nms_rotated(b, s, float(thr))
+    for seed in range(3):
+        g = torch.Generator().manual_seed(3000 + seed)
+        n, c, h, w = 2, 3 + seed, 17 + 5 * seed, 23
+        ph, pw, sr = [(7, 7, 0), (3, 5, 2), (2, 2, 3)][seed]
+        k = 19
+        rois = torch.cat([torch.randint(0, n, (k, 1), generator=g).float(),
+                          torch.rand(k, 2, generator=g) * torch.tensor([w * 4.0, h * 4.0]),
+                          2 + torch.rand(k, 2, generator=g) * 50, (torch.rand(k, 1, generator=g) - 0.5) * 360], 1)
+        x = torch.randn(n, c, h, w, generator=g)
+        y = D2.roi_align_rotated_forward(x, rois, 0.25, ph, pw, sr)
+        go = torch.randn(y.shape, generator=g)
+        out.update({f"sweep{seed}_cfg": np.asarray([ph, pw, sr]), f"sweep{seed}_x": x, f"sweep{seed}_rois": rois,
+                    f"sweep{seed}_y": y, f"sweep{seed}_go": go,
+                    f"sweep{seed}_gx": D2.roi_align_rotated_backward(go, rois, 0.25, ph, pw, n, c, h, w, sr)})
+    save("compiled_reference", **out)
+
+
+def gen_paste_masks_random():
+    """The reference's paste_masks_in_image on random masks and boxes inside a 150 x 200 image (the cross-check of
+    oracle/paste_ref.py in tests/test_oracle_pins.py)."""
+    spec = importlib.util.spec_from_file_location("ref_mask_ops", REF + "/detectron2/layers/mask_ops.py")
+    mo = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(mo)
+    g = torch.Generator().manual_seed(8)
+    masks = torch.rand(6, 28, 28, generator=g)
+    ctr = torch.rand(6, 2, generator=g) * torch.tensor([200.0, 150.0])
+    wh = 10 + torch.rand(6, 2, generator=g) * 90
+    boxes = torch.cat([ctr - wh / 2, ctr + wh / 2], 1)
+    save("paste_masks_random", masks=masks, boxes=boxes, hw=np.asarray([150, 200]),
+         out_bool=mo.paste_masks_in_image(masks, boxes, (150, 200), 0.5))
+
+
+def gen_reference_shim_protocol():
+    """The calls that the reference's deform-conv autograd Functions (detectron2/layers/deform_conv.py, `_DeformConv` and
+    `_ModulatedDeformConv`) make into `detectron2._C`, recorded through a stand-in module: which input goes into which
+    argument, the shape of every buffer the caller allocates and whether it is zero when passed, every scalar argument, and
+    which buffer each Function returns as its output or as each gradient.  tests/test_reference_shim.py replays the record
+    against the signatures of detectron2_b200._C."""
+    import json
+    import math
+    import types
+
+    class FakeCuda(torch.Tensor):  # the reference Functions refuse CPU tensors; they only test the flag
+        @property
+        def is_cuda(self):
+            return True
+
+    def fc(t):
+        return torch.Tensor._make_subclass(FakeCuda, t, t.requires_grad)
+
+    def plain(t):
+        return t.detach().as_subclass(torch.Tensor)
+
+    g = torch.Generator().manual_seed(0)
+    n, c, h, w, co = 2, 4, 7, 9, 6
+    inputs = {"x": torch.randn(n, c, h, w, generator=g), "off": torch.randn(n, 18, h, w, generator=g),
+              "mask": torch.sigmoid(torch.randn(n, 9, h, w, generator=g)),
+              "w": torch.randn(co, c, 3, 3, generator=g) * (1 / math.sqrt(c * 9)), "bias": torch.randn(co, generator=g),
+              "go": torch.randn(n, co, h, w, generator=g)}
+    calls, buffers = [], {}  # buffers: id(tensor) -> (buffer number, tensor kept alive so that ids stay unique)
+
+    def encode(a):
+        if not isinstance(a, torch.Tensor):
+            assert a is None or isinstance(a, (bool, int, float)), type(a)
+            return a
+        p = plain(a)
+        for name, t in inputs.items():
+            if p.shape == t.shape and torch.equal(p, t):
+                return {"input": name}
+        if id(a) not in buffers:
+            buffers[id(a)] = (len(buffers), a)
+        return {"buffer": buffers[id(a)][0], "shape": list(p.shape), "zero": bool((p == 0).all())}
+
+    def recorder(name):
+        def fn(*args, **kwargs):
+            assert not kwargs, (name, kwargs)
+            calls.append({"fn": name, "args": [encode(a) for a in args]})
+            for a in args:  # every buffer a call writes holds its buffer number + 1 afterwards: identifies what is returned
+                if isinstance(a, torch.Tensor) and id(a) in buffers and a.numel():
+                    with torch.no_grad():
+                        a.fill_(buffers[id(a)][0] + 1)
+            return 1
+        return fn
+
+    shim = types.ModuleType("detectron2._C")
+    for name in ("deform_conv_forward", "deform_conv_backward_input", "deform_conv_backward_filter",
+                 "modulated_deform_conv_forward", "modulated_deform_conv_backward"):
+        setattr(shim, name, recorder(name))
+    shim.get_cuda_version, shim.has_cuda, shim.get_compiler_version = (lambda: "CUDA"), (lambda: True), (lambda: "nvcc")
+
+    def stub(name, **attrs):
+        m = types.ModuleType(name)
+        m.__dict__.update(attrs)
+        sys.modules[name] = m
+        return m
+
+    for k in [k for k in sys.modules if k.startswith(("detectron2", "fvcore"))]:
+        del sys.modules[k]
+    fv = stub("fvcore", __version__="0.1.5")
+    fv.nn = stub("fvcore.nn")
+    stub("fvcore.nn.distributed", differentiable_all_reduce=lambda x: x)
+    fv.nn.weight_init = stub("fvcore.nn.weight_init")
+    sys.path.insert(0, REF)
+    import detectron2  # noqa: F401  (the real package __init__)
+
+    sys.modules["detectron2._C"] = shim
+    detectron2._C = shim
+    mod = importlib.import_module("detectron2.layers.deform_conv")
+
+    def returned(t):
+        v = plain(t).unique()
+        assert v.numel() == 1, "returned tensor is not one recorded buffer"
+        return int(v.item()) - 1
+
+    x, off, mask, wt, bias, go = (inputs[k] for k in ("x", "off", "mask", "w", "bias", "go"))
+    roles = {}
+    xs = [fc(t.clone().requires_grad_(True)) for t in (x, off, wt)]
+    y = mod.deform_conv(xs[0], xs[1], xs[2], 1, 1, 1, 1, 1, 64)
+    y.backward(fc(go))
+    roles["v1"] = dict(zip(("y", "x", "off", "w"), [returned(t) for t in [y] + [a.grad for a in xs]]))
+    xs = [fc(t.clone().requires_grad_(True)) for t in (x, off, mask, wt, bias)]
+    y = mod.modulated_deform_conv(xs[0], xs[1], xs[2], xs[3], xs[4], 1, 1, 1, 1, 1)
+    y.backward(fc(go))
+    roles["v2"] = dict(zip(("y", "x", "off", "mask", "w", "bias"), [returned(t) for t in [y] + [a.grad for a in xs]]))
+    save("reference_shim_protocol", protocol=np.asarray(json.dumps({"calls": calls, "returns": roles})), **inputs)
+
+
+GENERATORS = {"roi_align": gen_roi_align, "roi_align_rotated": gen_roi_align_rotated, "nms": gen_nms,
+              "rotated": gen_rotated_iou_nms, "deform_conv": gen_deform_conv, "paste_masks": gen_paste_masks,
+              "rpn_proposals": gen_rpn_proposals, "fast_rcnn_inference": gen_fast_rcnn_inference,
+              "retinanet_inference": gen_retinanet_inference, "postprocessing": gen_postprocessing,
+              "compiled_reference": gen_compiled_reference, "paste_masks_random": gen_paste_masks_random,
+              "reference_shim_protocol": gen_reference_shim_protocol}
+
 if __name__ == "__main__":
     torch.set_num_threads(1)
-    gen_roi_align()
-    gen_roi_align_rotated()
-    gen_nms()
-    gen_rotated_iou_nms()
-    gen_deform_conv()
-    gen_paste_masks()
-    gen_rpn_proposals()
-    gen_fast_rcnn_inference()
-    gen_retinanet_inference()
-    gen_postprocessing()
+    for name in sys.argv[1:] or list(GENERATORS):
+        GENERATORS[name]()

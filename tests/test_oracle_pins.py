@@ -4,7 +4,7 @@ Three layers of evidence (all CPU, `-m "not gpu"`):
   1. the reference's own known-answer tables (cited per test),
   2. the committed golden fixtures generated from torchvision CPU / the compiled reference CPU csrc /
      the reference python paste_masks (tests/golden/make_golden.py),
-  3. live cross-checks against torchvision CPU and oracle/_ref when they are loadable.
+  3. cross-checks against torchvision CPU (live) and the compiled reference CPU csrc (results stored by make_golden.py).
 """
 import math
 
@@ -224,27 +224,19 @@ def test_live_vs_torchvision():
         assert torch.equal(orc.nms(boxes, scores, thr), tv.ops.nms(boxes, scores, thr))
 
 
-def test_live_vs_compiled_reference():
-    if not orc.load_reference():
-        pytest.skip("oracle/_ref not available")
-    g = torch.Generator().manual_seed(11)
-    n = 150
-    b = torch.stack([torch.rand(n, generator=g) * 80, torch.rand(n, generator=g) * 80, 1 + torch.rand(n, generator=g) * 40,
-                     1 + torch.rand(n, generator=g) * 40, (torch.rand(n, generator=g) - 0.5) * 400], 1)
-    ref = torch.ops.detectron2.box_iou_rotated(b, b.flip(0))
+def test_live_vs_compiled_reference(golden):
+    """box_iou_rotated / nms_rotated against what the compiled reference csrc returned (fixture from make_golden.py)."""
+    d = golden("compiled_reference")
+    b, s = T(d["b"]), T(d["s"])
     got = orc.box_iou_rotated(b, b.flip(0))
-    assert np.array_equal(got.numpy().view(np.uint32), ref.numpy().view(np.uint32))
-    s = torch.rand(n, generator=g)
-    for thr in (0.2, 0.5):
-        assert torch.equal(orc.nms_rotated(b, s, thr), torch.ops.detectron2.nms_rotated(b, s, thr))
+    assert np.array_equal(got.numpy().view(np.uint32), d["ious"].view(np.uint32))
+    for i, thr in enumerate(d["thr"]):
+        assert torch.equal(orc.nms_rotated(b, s, float(thr)), T(d[f"keep{i}"]))
 
 
 def test_paste_port_matches_fixture_and_reference(golden):
-    """oracle/paste_ref.py (the CPU-baseline port) against the golden fixture, and against the real reference
-    function when /root/reference is present (authoring container)."""
-    import importlib.util
-    import os
-
+    """oracle/paste_ref.py (the CPU-baseline port) against the golden fixture, and against what the real reference
+    function returned on random masks and boxes (fixture from make_golden.py)."""
     from oracle import paste_ref
 
     d = golden("paste_masks")
@@ -252,18 +244,9 @@ def test_paste_port_matches_fixture_and_reference(golden):
     got = paste_ref.paste_masks_in_image_cpu(T(d["masks"]), T(d["boxes"]), (h, w), 0.5)
     keep = [i for i in range(9) if i != 1]  # box 1 is degenerate (x1 == x0): nan grid, not a baseline case
     assert torch.equal(got[keep], T(d["out_bool"])[keep])
-    path = "/root/reference/detectron2/layers/mask_ops.py"
-    if os.path.exists(path):
-        spec = importlib.util.spec_from_file_location("ref_mask_ops", path)
-        mo = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(mo)
-        g = torch.Generator().manual_seed(8)
-        masks = torch.rand(6, 28, 28, generator=g)
-        ctr = torch.rand(6, 2, generator=g) * torch.tensor([200.0, 150.0])
-        wh = 10 + torch.rand(6, 2, generator=g) * 90
-        boxes = torch.cat([ctr - wh / 2, ctr + wh / 2], 1)
-        assert torch.equal(paste_ref.paste_masks_in_image_cpu(masks, boxes, (150, 200), 0.5),
-                           mo.paste_masks_in_image(masks, boxes, (150, 200), 0.5))
+    d = golden("paste_masks_random")
+    h, w = [int(v) for v in d["hw"]]
+    assert torch.equal(paste_ref.paste_masks_in_image_cpu(T(d["masks"]), T(d["boxes"]), (h, w), 0.5), T(d["out_bool"]))
 
 
 def _rpn_fixture(golden):
@@ -327,18 +310,11 @@ def test_sweep_batched_nms_vs_torchvision(seed):
 
 
 @pytest.mark.parametrize("seed", range(3))
-def test_sweep_roi_align_rotated_vs_compiled_reference(seed):
-    if not orc.load_reference():
-        pytest.skip("oracle/_ref not available")
-    g = torch.Generator().manual_seed(3000 + seed)
-    n, c, h, w = 2, 3 + seed, 17 + 5 * seed, 23
-    ph, pw, sr = [(7, 7, 0), (3, 5, 2), (2, 2, 3)][seed]
-    k = 19
-    rois = torch.cat([torch.randint(0, n, (k, 1), generator=g).float(), torch.rand(k, 2, generator=g) * torch.tensor([w * 4.0, h * 4.0]),
-                      2 + torch.rand(k, 2, generator=g) * 50, (torch.rand(k, 1, generator=g) - 0.5) * 360], 1)
-    x = torch.randn(n, c, h, w, generator=g)
-    ref = torch.ops.detectron2.roi_align_rotated_forward(x, rois, 0.25, ph, pw, sr)
+def test_sweep_roi_align_rotated_vs_compiled_reference(seed, golden):
+    # inputs and the compiled reference's results stored by make_golden.py (gen_compiled_reference)
+    d = golden("compiled_reference")
+    ph, pw, sr = (int(v) for v in d[f"sweep{seed}_cfg"])
+    x, rois, ref, go, gref = (T(d[f"sweep{seed}_{k}"]) for k in ("x", "rois", "y", "go", "gx"))
+    n, c, h, w = x.shape
     assert torch.allclose(orc.roi_align_rotated_forward(x, rois, 0.25, ph, pw, sr), ref, rtol=1e-4, atol=1e-5)
-    go = torch.randn(ref.shape, generator=g)
-    gref = torch.ops.detectron2.roi_align_rotated_backward(go, rois, 0.25, ph, pw, n, c, h, w, sr)
     assert torch.allclose(orc.roi_align_rotated_backward(go, rois, 0.25, ph, pw, n, c, h, w, sr), gref, rtol=1e-4, atol=1e-4)

@@ -1,24 +1,20 @@
 """The `detectron2._C`-shaped deform-conv shim (detectron2_b200/_C.py, SURVEY.md 8b "pybind functions").
 
-CPU part (authoring container only, needs /root/reference): the REAL, unmodified reference autograd Functions
-`_DeformConv` / `_ModulatedDeformConv` (detectron2/layers/deform_conv.py:29-184, :205-313) are imported with our shim
-bound as `detectron2._C`.  They refuse CPU tensors, so the tensors are wrapped in a subclass that reports is_cuda, and the
-shim's five entry points are backed by the CPU oracle for this test: what is verified is the CALL PROTOCOL the reference
-uses against our signatures -- argument order (width-first for DCNv1), caller-allocated outputs written in place,
-gradients accumulated into zero-initialised buffers -- by comparing the reference Functions' results with torchvision
-autograd.  GPU part: the same protocol, restated call by call, against the real kernels.
+CPU part: the calls that the REAL, unmodified reference autograd Functions `_DeformConv` / `_ModulatedDeformConv`
+(detectron2/layers/deform_conv.py:29-184, :205-313) make into `detectron2._C` were recorded once from the reference
+(tests/golden/reference_shim_protocol.npz, written by tests/golden/make_golden.py) and are replayed here against a module
+with our shim's signatures whose five entry points are backed by the CPU oracle: what is verified is the CALL PROTOCOL the
+reference uses against our signatures -- argument order (width-first for DCNv1), caller-allocated outputs written in
+place, gradients accumulated into zero-initialised buffers -- by comparing the buffers the reference Functions return
+with torchvision autograd.  GPU part: the same protocol, restated call by call, against the real kernels.
 """
 import inspect
+import json
 import math
-import os
-import sys
 import types
 
 import pytest
 import torch
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
 
 
 class FakeCuda(torch.Tensor):
@@ -33,42 +29,7 @@ def _fc(t):
     return None if t is None else torch.Tensor._make_subclass(FakeCuda, t, t.requires_grad)
 
 
-def _import_reference_deform_conv(shim):
-    def stub(name, **attrs):
-        m = types.ModuleType(name)
-        m.__dict__.update(attrs)
-        sys.modules[name] = m
-        return m
-
-    saved = {k: v for k, v in sys.modules.items() if k.startswith(("detectron2", "fvcore"))}
-    for k in saved:
-        del sys.modules[k]
-    fv = stub("fvcore", __version__="0.1.5")
-    fv.nn = stub("fvcore.nn")
-    stub("fvcore.nn.distributed", differentiable_all_reduce=lambda x: x)
-    fv.nn.weight_init = stub("fvcore.nn.weight_init")
-    sys.path.insert(0, REF)
-    try:
-        import detectron2  # noqa: F401  (the real package __init__)
-
-        sys.modules["detectron2._C"] = shim
-        detectron2._C = shim
-        import importlib
-
-        mod = importlib.import_module("detectron2.layers.deform_conv")
-    finally:
-        sys.path.remove(REF)
-    return mod, saved
-
-
-def _restore(saved):
-    for k in [k for k in sys.modules if k.startswith(("detectron2", "fvcore"))]:
-        del sys.modules[k]
-    sys.modules.update(saved)
-
-
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (GPU box)")
-def test_reference_functions_drive_the_shim_signatures():
+def test_reference_functions_drive_the_shim_signatures(golden):
     import torchvision
 
     from detectron2_b200 import _C as real_shim
@@ -141,36 +102,41 @@ def test_reference_functions_drive_the_shim_signatures():
         setattr(shim, name, fn)
     shim.get_cuda_version, shim.has_cuda, shim.get_compiler_version = real_shim.get_cuda_version, real_shim.has_cuda, real_shim.get_compiler_version
 
-    mod, saved = _import_reference_deform_conv(shim)
-    try:
-        g = torch.Generator().manual_seed(0)
-        n, c, h, w, co = 2, 4, 7, 9, 6
-        x = torch.randn(n, c, h, w, generator=g)
-        off = torch.randn(n, 18, h, w, generator=g)
-        mask = torch.sigmoid(torch.randn(n, 9, h, w, generator=g))
-        wt = torch.randn(co, c, 3, 3, generator=g) * (1 / math.sqrt(c * 9))
-        bias = torch.randn(co, generator=g)
-        go = torch.randn(n, co, h, w, generator=g)
-        W_HOLDER[0] = wt
-        # ---- DCNv1 through the reference's _DeformConv
-        xs = [_fc(t.clone().requires_grad_(True)) for t in (x, off, wt)]
-        y = mod.deform_conv(xs[0], xs[1], xs[2], 1, 1, 1, 1, 1, 64)
-        y.backward(_fc(go))
-        ref = tv_all(x, off, None, wt, None, (1, 1), (1, 1), (1, 1), go)
-        assert torch.allclose(plain(y), tv_all(x, off, None, wt, None, (1, 1), (1, 1), (1, 1)), atol=1e-5)
-        for a, b in zip(xs, (ref[0], ref[1], ref[3])):
-            assert torch.allclose(plain(a.grad), b, atol=1e-5)
-        # ---- DCNv2 through the reference's _ModulatedDeformConv
-        xs = [_fc(t.clone().requires_grad_(True)) for t in (x, off, mask, wt, bias)]
-        y = mod.modulated_deform_conv(xs[0], xs[1], xs[2], xs[3], xs[4], 1, 1, 1, 1, 1)
-        y.backward(_fc(go))
-        ref = tv_all(x, off, mask, wt, bias, (1, 1), (1, 1), (1, 1), go)
-        for a, b in zip(xs, ref):
-            assert torch.allclose(plain(a.grad), b, atol=1e-5)
-        assert calls == ["deform_conv_forward", "deform_conv_backward_input", "deform_conv_backward_filter",
-                         "modulated_deform_conv_forward", "modulated_deform_conv_backward"]
-    finally:
-        _restore(saved)
+    # replay the calls the reference Functions made (tests/golden/make_golden.py, gen_reference_shim_protocol): the same
+    # arguments in the same positions, buffers allocated as the caller allocated them (NaN where it used new_empty)
+    d = golden("reference_shim_protocol")
+    protocol = json.loads(str(d["protocol"]))
+    inputs = {k: torch.from_numpy(d[k]) for k in ("x", "off", "mask", "w", "bias", "go")}
+    x, off, mask, wt, bias, go = (inputs[k] for k in ("x", "off", "mask", "w", "bias", "go"))
+    W_HOLDER[0] = wt
+    buffers = {}
+
+    def arg(a):
+        if isinstance(a, dict) and "input" in a:
+            return _fc(inputs[a["input"]].clone())
+        if isinstance(a, dict):
+            if a["buffer"] not in buffers:
+                fill = 0.0 if a["zero"] else math.nan
+                buffers[a["buffer"]] = _fc(torch.full(a["shape"], fill))
+            return buffers[a["buffer"]]
+        return a
+
+    for call in protocol["calls"]:
+        getattr(shim, call["fn"])(*[arg(a) for a in call["args"]])
+    assert calls == ["deform_conv_forward", "deform_conv_backward_input", "deform_conv_backward_filter",
+                     "modulated_deform_conv_forward", "modulated_deform_conv_backward"]
+    # ---- DCNv1 through the reference's _DeformConv
+    got = {k: plain(buffers[b]) for k, b in protocol["returns"]["v1"].items()}
+    assert torch.allclose(got["y"], tv_all(x, off, None, wt, None, (1, 1), (1, 1), (1, 1)), atol=1e-5)
+    ref = tv_all(x, off, None, wt, None, (1, 1), (1, 1), (1, 1), go)
+    for k, b in zip(("x", "off", "w"), (ref[0], ref[1], ref[3])):
+        assert torch.allclose(got[k], b, atol=1e-5), k
+    # ---- DCNv2 through the reference's _ModulatedDeformConv
+    got = {k: plain(buffers[b]) for k, b in protocol["returns"]["v2"].items()}
+    assert torch.allclose(got["y"], tv_all(x, off, mask, wt, bias, (1, 1), (1, 1), (1, 1)), atol=1e-5)
+    ref = tv_all(x, off, mask, wt, bias, (1, 1), (1, 1), (1, 1), go)
+    for k, b in zip(("x", "off", "mask", "w", "bias"), ref):
+        assert torch.allclose(got[k], b, atol=1e-5), k
 
 
 def test_shim_exports_the_reference_pybind_names():
